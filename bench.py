@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the 3DHumanGAN generator hot path on B200 (and its CPU reference arm).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload C2|C2native|C5|tiny]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload C2|C2native|C5|tiny] [--dump-outputs DIR]
 
 One "step" = one `Map3DGenerator.forward` over one batch of synthetic latents + random SMPL-like poses
 (train-mode BatchNorm, as the reference's trainer runs the generator) at BASELINE.json configs[1]:
@@ -14,6 +14,7 @@ batch 8 per GPU, 512x512, render 96x96, 32 samples per ray.  Prints ONE JSON lin
                measured peak in MEASURED_PEAKS.json
   cpu_baseline the CPU oracle (port of the reference's PyTorch path) on the host cores, bounded sample
   --impl reference   times that CPU arm on its own (rank 0 only)
+  --dump-outputs DIR after the timed steps, rank 0 writes what the timed path returned in its last step as DIR/<name>.npy
 
 Multi-GPU (`torchrun ... bench.py --gpus N`): weak scaling, 8 images per rank, SyncBatchNorm statistics
 all-reduced over NCCL inside the forward (18 small all-reduces), no other data-path collective.
@@ -37,6 +38,7 @@ sys.path.insert(0, ROOT)
 METRIC = "images_per_sec_G_fwd_512x512"
 UNIT = "images/s"
 FALLBACK_PEAKS = {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}
+DUMP_BYTES = 60 * 2 ** 20          # --dump-outputs writes at most this much data (headroom under 64 MB for the .npy headers)
 
 
 _REAL_STDOUT = None
@@ -80,6 +82,25 @@ def ncu_traffic(entry, workload):
     return None if d is None else d["dram_bytes_per_launch_mean_of_18"]
 
 
+def dump_outputs(path, outputs):
+    """Write every output as <path>/<name>.npy, float64 as float64 and anything else as float32.  When together they exceed
+    DUMP_BYTES, each array is replaced by the same fraction of its elements (flattened) at positions drawn from a fixed seed,
+    so that runs with the same arguments, on any build, write files that compare element for element."""
+    import numpy as np
+    arrays = {}
+    for name, v in outputs.items():
+        t = v.detach().cpu() if torch.is_tensor(v) else torch.as_tensor(v)
+        arrays[name] = (t.double() if t.dtype == torch.float64 else t.float()).numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            flat = a.reshape(-1)
+            keep = int(flat.size * DUMP_BYTES / total)
+            a = flat[np.sort(np.random.default_rng(0).choice(flat.size, keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def workload_cfg(pkg, name):
     cfg = pkg.configs.baseline_config(name)
     cfg["nerf_noise"] = 0.0
@@ -92,7 +113,7 @@ def workload_cfg(pkg, name):
 def cpu_sample(pkg, name, steps, warmup, sample_div=4):
     """Times `oracle.port.generator_forward` for ONE image on a 1/sample_div^2 sub-grid of the workload
     (gen and render resolutions divided by sample_div, same 32 samples per ray, same dims) and scales
-    by the pixel ratio.  Returns (images_per_sec, cores, description)."""
+    by the pixel ratio.  Returns (images_per_sec, cores, description, median seconds per pass, outputs of the last pass)."""
     from oracle import port
     cores = host_cores()
     torch.set_num_threads(cores)
@@ -111,7 +132,7 @@ def cpu_sample(pkg, name, steps, warmup, sample_div=4):
     with torch.no_grad():
         for i in range(warmup + steps):
             t0 = time.perf_counter()
-            port.generator_forward(params, z, cond, cfg, u, noise, training=True)
+            out = port.generator_forward(params, z, cond, cfg, u, noise, training=True)
             if i >= warmup:
                 times.append(time.perf_counter() - t0)
     times.sort()
@@ -120,7 +141,7 @@ def cpu_sample(pkg, name, steps, warmup, sample_div=4):
             f"{cfg['render_height']}x{cfg['render_width']}x{S} sub-grid ({frac:.4f} of the workload's pixels), "
             f"median of {len(times)} passes {t:.2f} s (min {times[0]:.2f}, max {times[-1]:.2f}), scaled by pixel count; fp32, "
             f"torch {torch.__version__}, {cores} threads = len(os.sched_getaffinity(0)) (os.cpu_count() = {os.cpu_count()})")
-    return frac / t, cores, desc, t
+    return frac / t, cores, desc, t, out
 
 
 def host_cores():
@@ -149,9 +170,11 @@ def run_reference(args, pkg):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(3, min(args.steps, 5))
+    steps = args.steps
     warm = 1
-    ips, cores, desc, t = cpu_sample(pkg, args.workload, steps, warm)
+    ips, cores, desc, t, out = cpu_sample(pkg, args.workload, steps, warm)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     cfg = workload_cfg(pkg, args.workload)
     line = {
         "impl": "reference", "metric": METRIC, "value": ips, "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
@@ -309,9 +332,12 @@ def run_gpu(args, pkg):
         os.environ.setdefault("TORCH_NCCL_ASYNC_ERROR_HANDLING", "0")   # the watchdog must not query events of a capturing stream
         dist.init_process_group("nccl", device_id=dev)
 
+    last = {}                         # what the module returned in the latest resident step (--dump-outputs)
+
     def step_resident():
         with torch.no_grad():
-            return G(z_d, cond_d, **kw)["rgbs"]
+            last.update(G(z_d, cond_d, **kw))
+        return last["rgbs"]
 
     def step_e2e():
         with torch.no_grad():
@@ -344,6 +370,8 @@ def run_gpu(args, pkg):
     sampler = ClockSampler(local) if rank == 0 else None
     ms_total = timed(step_resident, args.steps)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
 
     # Per-kernel device time: the same step launched eagerly with a CUDA-event pair around every launch of the
     # C ABI (a captured graph cannot carry timing events).  Also counts this library's launches per step.
@@ -447,7 +475,7 @@ def run_gpu(args, pkg):
 
     cpu = None
     if world == 1 and not args.no_cpu:
-        ips, cores, desc, _ = cpu_sample(pkg, args.workload, 3, 1)
+        ips, cores, desc, _, _ = cpu_sample(pkg, args.workload, 3, 1)
         cpu = {"value": ips, "unit": UNIT, "cores": cores, "kind": "port", "sample": desc}
 
     line = {
@@ -518,12 +546,13 @@ def run_gpu(args, pkg):
     _leave(world, G)
 
 
-def train_leg(args, pkg, dev, rank, world, B, steps, warm, precision, split):
+def train_leg(args, pkg, dev, rank, world, B, steps, warm, precision, split, dump=None):
     """BASELINE.json's second metric: one G+D training iteration (discriminator step, then generator step) per step through
     `train_step.Trainer` -- the mirror of the reference's PhaseTrainer (DDP wrappers with their gradient all-reduce over
     NCCL when world > 1, SyncBatchNorm statistics all-reduced inside the generator, five Adam groups, clip, EMA, R1 on its
     2-of-8 phase schedule).  B images per GPU per iteration, in `split` micro-batches (the reference's `batch_split`).
-    Returns the sub-object that goes into the JSON line (rank 0) or None."""
+    Returns the sub-object that goes into the JSON line (rank 0) or None.  With `dump`, the two losses of the last timed
+    iteration are written there (dump_outputs)."""
     import torch.distributed as dist
     abi = importlib.import_module("3dhumangan_b200.abi")
     gen = importlib.import_module("3dhumangan_b200.modules.generator")
@@ -550,8 +579,10 @@ def train_leg(args, pkg, dev, rank, world, B, steps, warm, precision, split):
     resident["cond"] = {k: v.to(dev) for k, v in cond_h.items()}
     loss_h = torch.empty(2).pin_memory()
 
+    last = []
+
     def step_resident():
-        return trainer.iteration(resident)
+        last[:] = trainer.iteration(resident)
 
     def step_e2e():
         batch = {k: v.to(dev, non_blocking=True) for k, v in host.items()}
@@ -592,6 +623,8 @@ def train_leg(args, pkg, dev, rank, world, B, steps, warm, precision, split):
     ms_total = timed(step_resident, steps, record=True)
     launches = abi.LAUNCHES
     clocks = sampler.stop() if sampler else None
+    if dump:
+        dump_outputs(dump, {"d_loss": last[0], "g_loss": last[1]})
     ms_e2e = timed(step_e2e, steps)
     finite = bool(torch.isfinite(loss_h).all())
     it_ms = [(r1, a.elapsed_time(b)) for r1, a, b in per_iter]
@@ -656,7 +689,8 @@ def run_train(args, pkg):
         os.environ.setdefault("NCCL_DEBUG", "WARN")
         dist.init_process_group("nccl", device_id=dev)
     abi.require_device()
-    leg = train_leg(args, pkg, dev, rank, world, args.train_batch, args.steps, max(args.warmup, 3), args.precision, args.train_split)
+    leg = train_leg(args, pkg, dev, rank, world, args.train_batch, args.steps, max(args.warmup, 3), args.precision, args.train_split,
+                    dump=args.dump_outputs if rank == 0 else None)
     if rank == 0:
         leg.update(higher_is_better=True, vs_baseline=None, data="synthetic", cpu_baseline=None)
         emit(leg)
@@ -693,7 +727,10 @@ def main():
     ap.add_argument("--train-batch", type=int, default=16, help="images per GPU per training iteration (config C3: 16)")
     ap.add_argument("--train-split", type=int, default=2, help="micro-batches per iteration (the reference's batch_split)")
     ap.add_argument("--train-steps", type=int, default=4, help="timed training iterations in the default run")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     claim_stdout()
     pkg = importlib.import_module("3dhumangan_b200")
     if args.impl == "reference":

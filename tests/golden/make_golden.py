@@ -39,6 +39,9 @@ CASES = {
                                  feature_dim=384), 7, 200.0, 1.0, 2, 0.5),
 }
 D_CASES = {"d_tiny": (dict(gen_height=64, gen_width=64), 7, 2)}
+# the g_tiny_dense recipe drawn at a second seed: the reference's own draws, which tests/test_oracle_pin.py replays through
+# `rng.draw_render_noise` (stored as <case>_seed<seed>.npz: rgbs, and of the feature maps every 17th element + the L2 norm)
+REPLAY = ("g_tiny_dense", 77)
 
 
 def reference_modules():
@@ -102,6 +105,13 @@ def main():
                             weight_u0=sd[blk + "conv_0.weight_u"].numpy())
         manifest[name] = {"rng_seed": seed, "recipe": [CASES[name][0], CASES[name][1], *CASES[name][2:]]}
         print(name, "rgbs", tuple(out["rgbs"].shape), float(out["rgbs"].abs().mean()))
+    name, seed = REPLAY
+    if not only or f"{name}_seed{seed}" in only:
+        cfg, params, cond, z, B = build_case(pkg, port, name)
+        out, fmap, _, _ = run_reference_generator(gens, impl, cfg, copy.deepcopy(params), cond, z, seed)
+        np.savez_compressed(os.path.join(HERE, f"{name}_seed{seed}.npz"), rgbs=out["rgbs"].numpy(),
+                            feature_maps_every17=fmap.reshape(-1)[::17].numpy(), feature_maps_norm=np.array(float(fmap.double().norm())))
+        print(f"{name}_seed{seed}", "rgbs", tuple(out["rgbs"].shape))
     for name, (over, pseed, B) in D_CASES.items():
         if only and name not in only:
             continue

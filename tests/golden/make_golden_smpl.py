@@ -17,7 +17,6 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "oracle", "shims"))
-sys.path.insert(0, "/root/reference")
 
 
 def inputs(seed=0, B=3, V=500, J=24, NB=10):
@@ -35,6 +34,7 @@ def inputs(seed=0, B=3, V=500, J=24, NB=10):
 
 
 def main():
+    sys.path.insert(0, os.environ["HG_REFERENCE"])           # a checkout of the reference
     from oracle import smpl_port as sp
     import lib.components.smpl as rsmpl
     for n in ("blend_shapes", "vertices2joints", "batch_rodrigues", "batch_rigid_transform"):

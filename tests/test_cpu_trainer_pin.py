@@ -1,125 +1,92 @@
-"""Host-side trainer logic pinned LIVE against the reference's own code (build container only: needs /root/reference; skipped on
-the GPU box): the five Adam parameter groups of `PhaseTrainer.init_optimizer` (phase_trainer.py:57-76) and the EMA update of
-`lib/components/ema.py:29-48`, executed by the unmodified reference functions on THIS package's modules (same parameter names
-by the state_dict contract)."""
+"""Host-side trainer logic pinned against the reference's own code: the five Adam parameter groups of
+`PhaseTrainer.init_optimizer` (phase_trainer.py:57-76), the EMA update of `lib/components/ema.py:29-48`, the R1 penalty, the
+D-step / G-step composition, the curricula and the bias_act activation table.  The unmodified reference functions were executed
+on the recipes of tests/golden/make_golden_trainer.py (on THIS package's modules where parameters matter: same parameter names
+by the state_dict contract); tests/golden/trainer_pins.{json,npz} hold what they computed."""
 import copy
-import importlib
+import importlib.util
+import json
 import os
-import sys
 import types
 
+import numpy as np
 import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("HG_REFERENCE", "/root/reference")
-
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "lib")), reason="needs the reference checkout")
+GOLD = os.path.join(ROOT, "tests", "golden")
 
 
-def _reference(modname):
-    for p in (os.path.join(ROOT, "oracle", "shims"), REF):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    return importlib.import_module(modname)
+def _load_recipes():
+    spec = importlib.util.spec_from_file_location("make_golden_trainer", os.path.join(GOLD, "make_golden_trainer.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
 
 
-def _modules(pkg):
-    gen = importlib.import_module("3dhumangan_b200.modules.generator")
-    disc = importlib.import_module("3dhumangan_b200.modules.discriminator")
-    cfg = pkg.configs.baseline_config("tiny")
-    torch.manual_seed(0)
-    return gen.Map3DGenerator(**cfg), disc.UNetDiscriminator(**cfg), cfg
+rec = _load_recipes()
 
 
-def test_optimizer_groups_match_phase_trainer_init_optimizer(pkg, tmp_path):
+@pytest.fixture(scope="module")
+def gold():
+    with open(os.path.join(GOLD, "trainer_pins.json")) as f:
+        js = json.load(f, object_hook=rec.decode_hook)
+    arrays = np.load(os.path.join(GOLD, "trainer_pins.npz"))
+    js.update({k: torch.from_numpy(arrays[k]) for k in arrays.files})
+    return js
+
+
+def test_optimizer_groups_match_phase_trainer_init_optimizer(pkg, gold):
     ts = importlib.import_module("3dhumangan_b200.train_step")
-    pt = _reference("lib.trainers.phase_trainer")
-    G, D, cfg = _modules(pkg)
-    meta = dict(cfg, gen_lr=2e-5, disc_lr=2e-4, betas=(0.0, 0.9),      # (0, 0.9) in configs/map3d.py; this torch wants two floats
-                weight_decay=0, appearance_codes_lr_mul=3.0, mapping_net_lr_mul=0.5,
-                neural_field_lr_mul=0.25)
-    me = types.SimpleNamespace(generator_ddp=G, discriminator_ddp=D, output_dir=str(tmp_path), device="cpu")
-    pt.PhaseTrainer.init_optimizer(me, meta)                       # the reference's own method, unmodified
+    G, D, cfg = rec.modules(pkg)
+    meta = dict(cfg, **rec.OPT_META)
     og, od = ts.make_optimizers(G, D, meta, fused=False)
     og_f, od_f = ts.make_optimizers(G, D, meta, fused=True)         # the multi-tensor optimiser keeps the same groups
+    gname = {id(p): n for n, p in G.named_parameters()}
+    dname = {id(p): n for n, p in D.named_parameters()}
     for mine in (og, og_f):
-        assert len(mine.param_groups) == len(me.optimizer_G.param_groups) == 5
-        for a, b in zip(mine.param_groups, me.optimizer_G.param_groups):
+        assert len(mine.param_groups) == len(gold["optimizer_G"]) == 5
+        for a, b in zip(mine.param_groups, gold["optimizer_G"]):
             assert a["name"] == b["name"]
             assert a["lr"] == pytest.approx(b["lr"], rel=0, abs=0) and tuple(a["betas"]) == tuple(b["betas"])
             assert a["weight_decay"] == b["weight_decay"] and a["eps"] == b["eps"]
-            assert [id(p) for p in a["params"]] == [id(p) for p in b["params"]], a["name"]      # same tensors, same order
+            assert [gname[id(p)] for p in a["params"]] == b["params"], a["name"]      # same tensors, same order
     for mine in (od, od_f):
-        a, b = mine.param_groups[0], me.optimizer_D.param_groups[0]
-        assert len(mine.param_groups) == 1 and a["lr"] == b["lr"] and tuple(a["betas"]) == tuple(b["betas"])
-        assert [id(p) for p in a["params"]] == [id(p) for p in b["params"]]
+        a, b = mine.param_groups[0], gold["optimizer_D"][0]
+        assert len(mine.param_groups) == len(gold["optimizer_D"]) == 1 and a["lr"] == b["lr"] and tuple(a["betas"]) == tuple(b["betas"])
+        assert [dname[id(p)] for p in a["params"]] == b["params"]
     # every generator parameter is in exactly one group
     ids = [id(p) for g in og.param_groups for p in g["params"]]
     assert len(ids) == len(set(ids)) == len(list(G.parameters()))
 
 
-def test_parameter_ema_matches_reference_ema(pkg):
+def test_parameter_ema_matches_reference_ema(pkg, gold):
     ts = importlib.import_module("3dhumangan_b200.train_step")
-    ema_ref = _reference("lib.components.ema")
-    G, _, _ = _modules(pkg)
-    G2 = copy.deepcopy(G)
-    a = ts.ParameterEMA(G.parameters(), decay=0.999)
-    b = ema_ref.ExponentialMovingAverage(G2.parameters(), decay=0.999)
-    gen = torch.Generator().manual_seed(3)
-    for step in range(12):                                          # the num_updates ramp (1+n)/(10+n) and the plateau
-        with torch.no_grad():
-            for p, q in zip(G.parameters(), G2.parameters()):
-                d = torch.randn(p.shape, generator=gen) * 0.01
-                p.add_(d)
-                q.add_(d)
-        a.update(list(G.parameters()))
-        b.update(list(G2.parameters()))
-        assert a.num_updates == b.num_updates
-    assert len(a.shadow_params) == len(b.shadow_params)
-    for s, t in zip(a.shadow_params, b.shadow_params):
-        assert torch.allclose(s, t, rtol=1e-6, atol=1e-8)
+    G, _, _ = rec.modules(pkg)
+    params = list(G.parameters())
+    a, counts = rec.ema_run(params, lambda ps: ts.ParameterEMA(ps, decay=rec.EMA_DECAY))
+    assert counts == gold["ema_num_updates"]
+    assert len(a.shadow_params) == gold["ema_shadow_count"]
+
+    def check(tensors):
+        sample, moments = rec.ema_summary(tensors)
+        assert torch.allclose(sample, gold["ema_sample"], rtol=1e-6, atol=1e-8)
+        assert torch.allclose(moments, gold["ema_moments"], rtol=1e-6, atol=1e-8)
+
+    check(a.shadow_params)
     # copy_to writes the averages into the parameters that require grad, in order
     a.copy_to(G.parameters())
-    b.copy_to(G2.parameters())
-    for p, q in zip(G.parameters(), G2.parameters()):
-        assert torch.allclose(p, q, rtol=1e-6, atol=1e-8)
+    check(list(G.parameters()))
 
 
 @pytest.mark.parametrize("gan_lambda", [1.0, 0.0])
-def test_r1_penalty_matches_phase_trainer(gan_lambda):
+def test_r1_penalty_matches_phase_trainer(gan_lambda, gold):
     """`train_step.r1_penalty` against the reference's `_calculate_r1_regularization` (phase_trainer.py:259-294) on a small
     differentiable stand-in for the discriminator: value and the gradient the penalty sends into the parameters (the double
     backward), with an enabled-style scale factor going through `scaler.scale` / `get_scale`."""
     ts = importlib.import_module("3dhumangan_b200.train_step")
-    pt = _reference("lib.trainers.phase_trainer")
-
-    class Scaler:                     # GradScaler's two calls used there, with a non-trivial scale
-        def scale(self, t):
-            return t * 1024.0
-
-        def get_scale(self):
-            return 1024.0
-
-    g = torch.Generator().manual_seed(9)
-    w1 = torch.randn(6, 3, 3, 3, generator=g, dtype=torch.float64) * 0.3
-    w2 = torch.randn(5, 6, 1, 1, generator=g, dtype=torch.float64) * 0.3
-    x0 = torch.randn(3, 3, 8, 8, generator=g, dtype=torch.float64)
-    meta = dict(gan_lambda=gan_lambda, segmentation_lambda=1.0, r1_lambda=0.25)
-
-    def run(fn):
-        a, b = w1.clone().requires_grad_(True), w2.clone().requires_grad_(True)
-        x = x0.clone().requires_grad_(True)
-        h = torch.nn.functional.leaky_relu(torch.nn.functional.conv2d(x, a, padding=1), 0.2)
-        seg = torch.nn.functional.conv2d(torch.tanh(h), b)
-        out = {"prediction": (h * h).mean(dim=(1, 2, 3)), "segments": seg}
-        pen = fn(x, out)
-        pen.backward()
-        return float(pen), a.grad.clone(), b.grad.clone() if b.grad is not None else torch.zeros_like(b)
-
-    me = types.SimpleNamespace(scaler=Scaler(), amp=False)
-    ref = run(lambda x, out: pt.PhaseTrainer._calculate_r1_regularization(me, x, out, {"do_r1": True}, meta))
-    got = run(lambda x, out: ts.r1_penalty(x, out, Scaler(), meta))
+    ref = (float(gold[f"r1_{gan_lambda}_value"]), gold[f"r1_{gan_lambda}_grad_a"], gold[f"r1_{gan_lambda}_grad_b"])
+    got = rec.r1_run(ts.r1_penalty, gan_lambda)
     assert got[0] == pytest.approx(ref[0], rel=1e-12, abs=1e-18)
     assert torch.allclose(got[1], ref[1], rtol=1e-10, atol=1e-16) and torch.allclose(got[2], ref[2], rtol=1e-10, atol=1e-16)
     if gan_lambda > 0:
@@ -130,108 +97,42 @@ def test_r1_penalty_matches_phase_trainer(gan_lambda):
 # the composition of the two steps: the reference's own `_train_discriminator` / `_train_generator` (phase_trainer.py:344-560),
 # unmodified, against `train_step.Trainer.train_discriminator / train_generator` on the same stand-in networks
 # ----------------------------------------------------------------------------------------------------------------------
-class _StandInG(torch.nn.Module):
-    """A generator with the call signature the trainer uses (z, conditions, latent_indices=..., **meta) -> {'rgbs', 'rgbs_render'}."""
-
-    def __init__(self, L):
-        super().__init__()
-        g = torch.Generator().manual_seed(21)
-        self.neural_field_mapping_network = torch.nn.Linear(L, 6)
-        self.synthesis_network = torch.nn.Conv2d(6, 3, 3, padding=1)
-        with torch.no_grad():
-            for p in self.parameters():
-                p.copy_(torch.randn(p.shape, generator=g) * 0.3)
-
-    def forward(self, z, conditions, latent_indices=None, disable_synthesis=False, **kwargs):
-        h = torch.tanh(self.neural_field_mapping_network(z))[:, :, None, None] + conditions["x"]
-        rgb = torch.tanh(self.synthesis_network(h))
-        return {"rgbs": rgb, "rgbs_render": torch.nn.functional.avg_pool2d(rgb, 2)}
-
-
-class _StandInD(torch.nn.Module):
-    def __init__(self, label_dim):
-        super().__init__()
-        g = torch.Generator().manual_seed(22)
-        self.c1 = torch.nn.Conv2d(3, 8, 3, padding=1)
-        self.seg = torch.nn.Conv2d(8, label_dim, 1)
-        self.pred = torch.nn.Linear(8, 1)
-        self.step = 0
-        with torch.no_grad():
-            for p in self.parameters():
-                p.copy_(torch.randn(p.shape, generator=g) * 0.3)
-
-    def forward(self, x, conditions, alpha=1.0, mode="real", **kwargs):
-        h = torch.nn.functional.leaky_relu(self.c1(x), 0.2) + (0.1 if mode == "real" else -0.1) * conditions["x"][:, :1]
-        return {"prediction": self.pred(h.mean(dim=(2, 3))), "segments": self.seg(h), "latents": h.mean(dim=(2, 3))}
-
-
 @pytest.mark.parametrize("gan_lambda,do_r1", [(0.0, False), (0.0, True), (1.0, True)])
-def test_step_composition_matches_phase_trainer(pkg, gan_lambda, do_r1, monkeypatch):
+def test_step_composition_matches_phase_trainer(pkg, gan_lambda, do_r1, gold):
     ts = importlib.import_module("3dhumangan_b200.train_step")
-    pt = _reference("lib.trainers.phase_trainer")
-    L, LD, B, H = 5, 7, 4, 8
-    phase = {"name": "uncond", "uncond": True, "rotate": True, "gen_modal": "rgbs", "do_r1": do_r1}
-    meta = dict(latent_dim=L, label_dim=LD, z_dist="gaussian", gan_lambda=gan_lambda, segmentation_lambda=1.0, latent_lambda=0,
-                perceptual_lambda=[0, 0, 0, 0], photometric_lambda=0, r1_lambda=0.25, grad_clip=1e9, gen_lr=0.0, disc_lr=0.0,
-                betas=(0.0, 0.9), weight_decay=0, appearance_codes_lr_mul=1.0, mapping_net_lr_mul=1.0, neural_field_lr_mul=1.0,
-                batch_split=2, phases=[phase], render_height=4, render_width=4, gen_height=H, gen_width=H)
-    g = torch.Generator().manual_seed(23)
-    images = torch.randn(B, 3, H, H, generator=g).clamp_(-1, 1)
-    labels = torch.randint(0, LD, (B, H, H), generator=g)
-    x = torch.randn(B, 6, H, H, generator=g) * 0.2
-    z_d, z_g = torch.randn(B, L, generator=g), torch.randn(B, L, generator=g)
-
-    # ---- the reference's methods on a bare namespace
-    Gr, Dr = _StandInG(L), _StandInD(LD)
-    me = types.SimpleNamespace(amp=False, device="cpu", batch_split=2, rank=0, generator_ddp=Gr, discriminator_ddp=Dr, discriminator=Dr,
-                               scaler=torch.amp.GradScaler("cuda", enabled=False))
-    for name in ("_train_discriminator", "_train_generator", "_get_disc_input_real", "_get_disc_input_gen",
-                 "_calculate_r1_regularization", "_calculate_segmentation_loss"):
-        setattr(me, name, types.MethodType(getattr(pt.PhaseTrainer, name), me))
-    zs = [z_d, z_g]
-    monkeypatch.setattr(pt, "z_sampler", lambda *a, **k: zs.pop(0))
-    monkeypatch.setattr(pt.training_stats, "report", lambda *a, **k: None)
-    data = {"images": images, "body_segments": labels, "rasterized_segments": labels, "latents": torch.zeros(B, L), "x": x}
-    d_ref = me._train_discriminator(data, 1.0, meta, phase)
-    d_ref.backward()
-    dgrads = [p.grad.clone() for p in Dr.parameters()]
-    Gr.zero_grad()
-    Dr.zero_grad()
-    g_ref, _ = me._train_generator(data, 1.0, meta, phase)
-    ggrads = [p.grad.clone() for p in Gr.parameters()]
-
-    # ---- this package's trainer on identical stand-ins
-    Gm, Dm = _StandInG(L), _StandInD(LD)
+    L, LD, meta, phase, images, labels, x, z_d, z_g = rec.composition_case(gan_lambda, do_r1)
+    key = rec.composition_key(gan_lambda, do_r1)
+    Gm, Dm = rec.StandInG(L), rec.StandInD(LD)
+    dgrads = [gold[f"{key}_d_grad_{i}"] for i in range(len(list(Dm.parameters())))]
+    ggrads = [gold[f"{key}_g_grad_{i}"] for i in range(len(list(Gm.parameters())))]
     t = ts.Trainer(Gm, Dm, meta, amp=False, ddp=False, fused=False)
     batch = dict(images=images, labels=labels, cond={"x": x}, z_d=z_d, z_g=z_g)
     d_mine = t.train_discriminator(batch)
     for p, r in zip(Dm.parameters(), dgrads):
         assert torch.allclose(p.grad, r, rtol=1e-5, atol=1e-7), float((p.grad - r).abs().max())
-    assert float(d_mine) == pytest.approx(float(d_ref), rel=1e-6)
+    assert float(d_mine) == pytest.approx(float(gold[key + "_d_loss"]), rel=1e-6)
     g_mine = t.train_generator(batch)
     for p, r in zip(Gm.parameters(), ggrads):
         assert torch.allclose(p.grad, r, rtol=1e-5, atol=1e-7), float((p.grad - r).abs().max())
-    assert float(g_mine) == pytest.approx(float(g_ref), rel=1e-6, abs=1e-12)
+    assert float(g_mine) == pytest.approx(float(gold[key + "_g_loss"]), rel=1e-6, abs=1e-12)
     # learning rate 0, no clipping: both steps ran their optimiser / EMA tail without moving a parameter
-    for p, q in zip(list(Gm.parameters()) + list(Dm.parameters()), list(Gr.parameters()) + list(Dr.parameters())):
-        assert torch.equal(p.detach(), q.detach())
+    for i, p in enumerate(list(Gm.parameters()) + list(Dm.parameters())):
+        assert torch.equal(p.detach(), gold[f"{key}_param_{i}"])
 
 
 @pytest.mark.parametrize("name", ["MAP3DBN", "MAP3DBN512", "MAP3DBN512L"])
-def test_curricula_match_reference_configs(pkg, name):
+def test_curricula_match_reference_configs(pkg, name, gold):
     """`3dhumangan_b200.configs` (the drop-in `configs` package) against the reference's `configs/map3d.py` + `extract_metadata`
     (configs/__init__.py) for every shipped curriculum at steps on both sides of every schedule boundary."""
-    ref = _reference("configs")
-    mine = pkg.configs
-    cur_r, cur_m = getattr(ref, name), getattr(mine, name)
-    steps = sorted({0, 1, 999, 1000, 200000, 200001, 300000, 300001, 300002, 10 ** 6} | {int(k) for k in cur_r if isinstance(k, int)} |
-                   {int(k) + 1 for k in cur_r if isinstance(k, int)})
-    for step in steps:
-        a, b = ref.extract_metadata(cur_r, step), mine.extract_metadata(cur_m, step)
+    cur_m = getattr(pkg.configs, name)
+    ref = gold["curricula"][name]
+    for step, i in ref["steps"]:
+        a = ref["metadata"][i]
+        b = pkg.configs.extract_metadata(cur_m, step)
         for k, v in a.items():
             assert k in b, (name, step, k)
             if k == "neural_field_cls":
-                assert (v if isinstance(v, str) else v.__name__) == (b[k] if isinstance(b[k], str) else b[k].__name__)
+                assert v == (b[k] if isinstance(b[k], str) else b[k].__name__)
             else:
                 assert b[k] == v, (name, step, k, v, b[k])
         extra = set(b) - set(a)
@@ -243,7 +144,7 @@ def test_trainer_refuses_the_branches_it_does_not_mirror():
     meta = dict(latent_dim=5, label_dim=7, gan_lambda=0.0, segmentation_lambda=1.0, r1_lambda=0.0, grad_clip=1.0, gen_lr=0.0, disc_lr=0.0,
                 betas=(0.0, 0.9), weight_decay=0, appearance_codes_lr_mul=1.0, mapping_net_lr_mul=1.0, neural_field_lr_mul=1.0,
                 phases=[{"name": "uncond", "uncond": True, "rotate": True, "gen_modal": "rgbs_render", "do_r1": False}])
-    t = ts.Trainer(_StandInG(5), _StandInD(7), meta, amp=False, ddp=False, fused=False)
+    t = ts.Trainer(rec.StandInG(5), rec.StandInD(7), meta, amp=False, ddp=False, fused=False)
     batch = dict(images=torch.zeros(2, 3, 8, 8), labels=torch.zeros(2, 8, 8, dtype=torch.long), cond={"x": torch.zeros(2, 6, 8, 8)})
     with pytest.raises(RuntimeError, match="not built"):
         t.train_discriminator(batch)
@@ -251,36 +152,32 @@ def test_trainer_refuses_the_branches_it_does_not_mirror():
         t.train_generator(batch)
 
 
-def test_activation_table_matches_reference_bias_act():
+def test_activation_table_matches_reference_bias_act(gold):
     """ops/bias_act.ACTIVATIONS (id, default alpha, default gain, which tensor the backward keeps, second derivative) against the
     reference's `activation_funcs` (lib/components/ops/bias_act.py:22-32) -- the ids are what the C ABI's `act` argument means."""
     mine = importlib.import_module("3dhumangan_b200.ops.bias_act").ACTIVATIONS
-    ref = _reference("lib.components.ops.bias_act").activation_funcs
-    cuda_acts = {k: v for k, v in ref.items() if v.cuda_idx is not None}
+    cuda_acts = gold["activations"]
     assert set(mine) == set(cuda_acts)
-    for k, spec in cuda_acts.items():
+    for k, (cuda_idx, def_alpha, def_gain, ref, has_2nd_grad) in cuda_acts.items():
         aid, alpha, gain, keep, second = mine[k]
-        assert aid == spec.cuda_idx and alpha == pytest.approx(spec.def_alpha) and gain == pytest.approx(float(spec.def_gain))
-        assert keep == spec.ref and second == spec.has_2nd_grad
+        assert aid == cuda_idx and alpha == pytest.approx(def_alpha) and gain == pytest.approx(def_gain)
+        assert keep == ref and second == has_2nd_grad
 
 
-@pytest.mark.parametrize("tune,variant", [("", 0), ("lr", 0), ("lr", 3), ("map3d_mode", 0), ("map3d_mode", 2)])
-def test_get_config_matches_reference(pkg, tune, variant):
+@pytest.mark.parametrize("tune,variant", rec.GET_CONFIG)
+def test_get_config_matches_reference(pkg, tune, variant, gold):
     """`configs.get_config(opt)` (configs/__init__.py:49-76: curriculum lookup, neural-field class resolution, the two `--tune`
-    sweeps) on deep copies of both packages' curricula."""
-    ref = _reference("configs")
+    sweeps) on a deep copy of the package's curriculum."""
+    a = next(e for e in gold["get_config"] if e["tune"] == tune and e["variant"] == variant)
     mine = pkg.configs
-    name = "MAP3DBN512"
-    saved_r, saved_m = copy.deepcopy(getattr(ref, name)), copy.deepcopy(getattr(mine, name))
+    name = rec.GET_CONFIG_NAME
+    saved_m = copy.deepcopy(getattr(mine, name))
     try:
         opt = types.SimpleNamespace(config=name, tune=tune, variant=variant)
-        a, b = ref.get_config(opt), mine.get_config(opt)
+        b = mine.get_config(opt)
         assert a["name"] == b["name"] and a["map3d_mode"] == b["map3d_mode"]
-        assert a["neural_field_cls"].__name__ == b["neural_field_cls"].__name__
-        for k in a:
-            if isinstance(k, int):
-                assert a[k] == b[k], (k, a[k], b[k])
+        assert a["neural_field_cls"] == b["neural_field_cls"].__name__
+        for k, v in a["stages"]:
+            assert v == b[k], (k, v, b[k])
     finally:
-        setattr(ref, name, saved_r)
-        ref.__dict__[name] = saved_r
         setattr(mine, name, saved_m)
