@@ -86,6 +86,7 @@ SIGNATURES = {
     "hg_smpl_skin": (c_int, [c_void_p, c_long, c_void_p, c_void_p, c_int, c_void_p, c_long, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "hg_spectral_entry_bytes": (c_int, []),
     "hg_spectral_norm": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_float, c_void_p]),
+    "hg_mesh_raster": (c_int, [c_void_p] * 4 + [c_float] + [c_int] * 5 + [c_void_p] * 9),
 }
 
 

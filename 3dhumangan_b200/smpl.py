@@ -129,15 +129,24 @@ def _euler_xyz(e):
 
 
 @torch.no_grad()
-def cam2world_fix_body(cond, h_rotation, v_rotation, r_rotation):
-    """The view rotation of `SHHQPreprocessor._forward_fix_body` (preprocessor.py:72-98) -> cam2world [B,4,4]."""
+def body_rotation(cond, h_rotation, v_rotation, r_rotation):
+    """root rotation @ Euler XYZ of the view (preprocessor.py:80-87) -> [B,3,3]; its inverse is the rasteriser's R."""
+    dev = cond["R"].device
+    B = cond["R"].shape[0]
+    euler = torch.zeros(B, 3, dtype=torch.float32, device=dev)
+    euler[:, 1] = -torch.as_tensor(h_rotation, dtype=torch.float32, device=dev)
+    euler[:, 0] = math.pi - torch.as_tensor(v_rotation, dtype=torch.float32, device=dev)
+    euler[:, 2] = -torch.as_tensor(r_rotation, dtype=torch.float32, device=dev)
+    return cond["full_pose"][:, 0] @ _euler_xyz(euler)
+
+
+@torch.no_grad()
+def cam2world_fix_body(cond, h_rotation, v_rotation, r_rotation, Rb=None):
+    """The view rotation of `SHHQPreprocessor._forward_fix_body` (preprocessor.py:72-98) -> cam2world [B,4,4].
+    `Rb`: `body_rotation(cond, h, v, r)` when the caller has it already."""
     R, T = cond["R"], cond["T"]
-    B = R.shape[0]
-    euler = torch.zeros(B, 3, dtype=torch.float32, device=R.device)
-    euler[:, 1] = -torch.as_tensor(h_rotation, dtype=torch.float32, device=R.device)
-    euler[:, 0] = math.pi - torch.as_tensor(v_rotation, dtype=torch.float32, device=R.device)
-    euler[:, 2] = -torch.as_tensor(r_rotation, dtype=torch.float32, device=R.device)
-    Rb = cond["full_pose"][:, 0] @ _euler_xyz(euler)
+    if Rb is None:
+        Rb = body_rotation(cond, h_rotation, v_rotation, r_rotation)
     body = F.pad(Rb, (0, 1, 0, 1))
     body[:, -1, -1] = 1.0
     return torch.inverse(torch.bmm(torch.bmm(R, T), body).float())

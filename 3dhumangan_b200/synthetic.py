@@ -136,3 +136,61 @@ def make_conditions(batch_size: int, seed: int = 1, pose_std: float = 0.3, view_
         "intrinsics": f32(K),
         "scales": f32(torch.full((B,), scale, dtype=torch.float64)),
     }
+
+
+def make_body_mesh(seed: int = 0):
+    """A closed genus-0 body-like surface with SMPL's counts, for the preprocessor's rasteriser (`raster.py`).
+
+    A UV sphere of 82 rings x 84 segments + 2 poles has exactly V = 6 890 vertices and F = 13 776 faces.  It is stretched to a
+    body's proportions (y up, head at +y, like SMPL's template) and its radius is modulated by seeded waves and signed Gaussian
+    bumps, so the surface is not convex and a rotated view has real self-occlusions.  Faces are labelled over 24 classes by
+    height band (12) x side (2) of their centroid, standing in for `densepose_data.json`'s face labels.
+
+    -> dict(vertices [V,3] float32, faces [F,3] int64, faces_to_labels [F] int64, smpl=dict(v_template, shapedirs [V,3,10],
+    posedirs [207, V*3], J_regressor [24,V], parents [24], lbs_weights [V,24])); `smpl.SMPLModel.from_arrays(**mesh["smpl"])`
+    skins it with smooth blend shapes and distance-based weights around `_REST`'s joints.  Pure CPU torch, seeded."""
+    gen = torch.Generator().manual_seed(seed)
+    rings, segs = 82, 84
+    theta = math.pi * torch.arange(1, rings + 1, dtype=torch.float64) / (rings + 1)
+    phi = 2 * math.pi * torch.arange(segs, dtype=torch.float64) / segs
+    th, ph = theta[:, None].expand(rings, segs).reshape(-1), phi[None].expand(rings, segs).reshape(-1)
+    th = torch.cat([torch.zeros(1, dtype=torch.float64), th, torch.full((1,), math.pi, dtype=torch.float64)])
+    ph = torch.cat([torch.zeros(1, dtype=torch.float64), ph, torch.zeros(1, dtype=torch.float64)])
+    n = torch.stack([torch.sin(th) * torch.cos(ph), torch.cos(th), torch.sin(th) * torch.sin(ph)], -1)
+    p = torch.rand(4, generator=gen, dtype=torch.float64) * 2 * math.pi
+    r = 1.0 + 0.15 * torch.sin(3 * ph + p[0]) * torch.sin(2 * th) + 0.1 * torch.cos(5 * th + p[1]) \
+        + 0.06 * torch.sin(7 * ph + p[2]) * torch.sin(th) ** 2
+    centres = torch.nn.functional.normalize(torch.randn(14, 3, generator=gen, dtype=torch.float64), dim=-1)
+    amp = (torch.rand(14, generator=gen, dtype=torch.float64) - 0.4) * 0.7            # mostly outward bumps, some dents
+    r = r + (amp * torch.exp(-(1 - n @ centres.T) / 0.02)).sum(-1)
+    verts = n * r[:, None] * torch.tensor([0.32, 0.85, 0.17], dtype=torch.float64) + torch.tensor([0.0, -0.4, 0.0], dtype=torch.float64)
+
+    V = 2 + rings * segs
+    ring = lambda k, j: 1 + k * segs + j % segs
+    j = torch.arange(segs)
+    faces = [torch.stack([torch.zeros_like(j), ring(0, j), ring(0, j + 1)], -1)]
+    for k in range(rings - 1):
+        a, b, c, d = ring(k, j), ring(k, j + 1), ring(k + 1, j), ring(k + 1, j + 1)
+        faces += [torch.stack([a, c, b], -1), torch.stack([b, c, d], -1)]
+    faces.append(torch.stack([torch.full_like(j, V - 1), ring(rings - 1, j + 1), ring(rings - 1, j)], -1))
+    faces = torch.cat(faces).to(torch.int64)
+    cen = verts[faces].mean(1)
+    y0, y1 = verts[:, 1].min(), verts[:, 1].max()
+    band = ((cen[:, 1] - y0) / (y1 - y0) * 12).floor().clamp(0, 11).to(torch.int64)
+    labels = band * 2 + (cen[:, 0] > 0).to(torch.int64)
+
+    rest = torch.tensor(_REST, dtype=torch.float64)
+    d = torch.cdist(verts, rest)
+    w = torch.softmax(-d / 0.08, dim=-1)
+    top = torch.topk(w, 4, dim=-1)
+    lbs = torch.zeros_like(w).scatter_(1, top.indices, top.values)
+    lbs = lbs / lbs.sum(-1, keepdim=True)
+    jreg = torch.softmax(-d.T / 0.05, dim=-1)
+    wave = lambda k: torch.sin(verts @ (torch.randn(3, k, generator=gen, dtype=torch.float64) * 3)
+                               + torch.rand(k, generator=gen, dtype=torch.float64) * 2 * math.pi)
+    shapedirs = 0.02 * wave(30).reshape(V, 10, 3).transpose(1, 2)
+    posedirs = 0.003 * wave(207 * 3).reshape(V, 207, 3).permute(1, 0, 2).reshape(207, V * 3)
+    f32 = lambda t: t.to(torch.float32).contiguous()
+    return {"vertices": f32(verts), "faces": faces, "faces_to_labels": labels,
+            "smpl": dict(v_template=f32(verts), shapedirs=f32(shapedirs), posedirs=f32(posedirs), J_regressor=f32(jreg),
+                         parents=torch.tensor(_PARENTS, dtype=torch.int64), lbs_weights=f32(lbs))}

@@ -275,6 +275,19 @@ int hg_smpl_pose(const float* jpart, int nblk, const float* pose, int pose_is_ro
 int hg_smpl_skin(const float* v_in, long v_bstride, const float* feat, const float* posedirs, int P, const float* lbs_weights,
                  long w_bstride, const float* A, float* verts, int B, int V, int J, void* stream);
 
+/* ---- the preprocessor's mesh rasteriser (SURVEY.md 8f-2) --------------------------------------------------------------------
+ * Replaces pytorch3d's MeshRasterizer (faces_per_pixel 1, blur_radius 0, no culling, perspective-correct) as called by
+ * SHHQPreprocessor._forward_rasterize (lib/data/preprocessor.py:138-152) and the label / semantic look-ups after it (:154-174).
+ * verts [B,V,3]; faces [F,3] int32 in [0,V) (NOT checked here), shared by the batch; R [B,3,3], T [B,3]: view = X @ R + T;
+ * focal: in-NDC focal length (the reference passes -1/tan(0.5 deg)).  keys [B,H,W] uint64 workspace (cleared here).
+ * Outputs, each optional (NULL = not written): pix_to_face [B,H,W] int64 packed b*F + face, -1 background; zbuf [B,H,W] and
+ * bary [B,H,W,3] (perspective-correct), -1 background; segments [B,H,W] int64 = faces_to_labels[face] + 2, background 1;
+ * semantics [B,3,H,W] = sem_verts[V,3] at the face vertex of the largest barycentric (first maximum), background 0.
+ * The arithmetic is oracle/raster_port.py's, bit for bit; deterministic (lowest face on equal depth). */
+int hg_mesh_raster(const float* verts, const int* faces, const float* R, const float* T, float focal, int B, int V, int F, int H,
+                   int W, unsigned long long* keys, const long* faces_to_labels, const float* sem_verts, long* pix_to_face,
+                   float* zbuf, float* bary, long* segments, float* semantics, void* stream);
+
 /* ---- loss + optimiser tail of a training iteration (SURVEY.md 8f-1) ---------------------------------------------------
  * Class-balanced segmentation cross entropy, PhaseTrainer._calculate_segmentation_loss mode 'cross_entropy_balanced'
  * (lib/trainers/phase_trainer.py:203-256): histogram of the int64 labels -> per-class coefficients (numel / (occ * n_occ) *
