@@ -82,7 +82,7 @@ struct SpadeArgs {
   float* rgb_out;        // [B,3,HW]
   int B, HW, Hg, Wg, Rh, Rw;
   // generalisations used by the backward schedule (defaults reproduce the forward half-block):
-  int nkc;               // K chunks of 64 input channels per tile: 2, 4 or 8
+  int nkc;               // K chunks of 64 input channels per tile: 1, 2, 4 or 8
   int xC;                // channels per source tile (128 or 256); chunks beyond xC/64 come from x2
   const float* x2;       // second source [B,T,xC,128] (K = 512 products) or null
   float slope;           // operand LeakyReLU slope (1 = identity); backward epilogue: slope of the mask (0.2 / 0 = ReLU)
@@ -1169,6 +1169,8 @@ int hg_blocked_conv_wide(const float* x, const float* x2, const float* mod, cons
                          int passes, void* stream) {
   HG_REQUIRE(x && wimg && bias && out, "hg_blocked_conv_wide: null pointer");
   HG_REQUIRE(act == 0 || act == 1, "hg_blocked_conv_wide: act must be 0 (LeakyReLU(slope)) or 1 (sine)");
+  HG_REQUIRE(slope >= 0.f && slope <= 1.f, "hg_blocked_conv_wide: the operand computes LeakyReLU as max(v, slope*v), "
+             "which needs 0 <= slope <= 1 (got %g)", static_cast<double>(slope));
   HG_REQUIRE(!mod2 || (mod && x2), "hg_blocked_conv_wide: mod2 needs mod and a second source");
   HG_REQUIRE(!rgb_w || (rgb_b && rgb_out), "hg_blocked_conv_wide: rgb_b / rgb_out missing");
   HG_REQUIRE(passes == 1 || passes == 3, "hg_blocked_conv_wide: passes must be 1 or 3");

@@ -328,13 +328,14 @@ __global__ void __launch_bounds__(256) spade_combine_kernel(CombineArgs a) {
                             : make_float4(p < a.HW ? src[0] : 0.f, p + 1 < a.HW ? src[1] : 0.f, p + 2 < a.HW ? src[2] : 0.f, 0.f);
       }
     }
-    const float m0 = p < a.HW ? 1.f : 0.f, m1 = p + 1 < a.HW ? 1.f : 0.f, m2 = p + 2 < a.HW ? 1.f : 0.f,
-                m3 = p + 3 < a.HW ? 1.f : 0.f;
+    // padding rows (past HW) are SELECTED away, not multiplied by 0: the producers never write them, so they may hold NaN
+    const bool m0 = p < a.HW, m1 = p + 1 < a.HW, m2 = p + 2 < a.HW, m3 = p + 3 < a.HW;
 #pragma unroll 4
     for (int c = warp; c < kWC; c += 8) {
       float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
       float4 xv = make_float4(0.f, 0.f, 0.f, 0.f);
       if (a.ak || a.drgb) xv = __ldcs(reinterpret_cast<const float4*>(a.x + xoff + c * 128));
+      xv = make_float4(m0 ? xv.x : 0.f, m1 ? xv.y : 0.f, m2 ? xv.z : 0.f, m3 ? xv.w : 0.f);
       if (a.dpre) {
         const float4 d = __ldcs(reinterpret_cast<const float4*>(a.dpre + off + c * 128));
         const float g = a.g1[static_cast<long>(b) * 2 * kWC + c];
@@ -354,7 +355,7 @@ __global__ void __launch_bounds__(256) spade_combine_kernel(CombineArgs a) {
         for (int j = 0; j < 3; ++j) {
           const float w = s_wrgb[j * kWC + c];
           v.x = fmaf(w, r[j].x, v.x); v.y = fmaf(w, r[j].y, v.y); v.z = fmaf(w, r[j].z, v.z); v.w = fmaf(w, r[j].w, v.w);
-          t[j] = (r[j].x * xv.x * m0 + r[j].y * xv.y * m1) + (r[j].z * xv.z * m2 + r[j].w * xv.w * m3);
+          t[j] = (r[j].x * xv.x + r[j].y * xv.y) + (r[j].z * xv.z + r[j].w * xv.w);
         }
         if (a.dwrgb) {
 #pragma unroll
@@ -370,7 +371,7 @@ __global__ void __launch_bounds__(256) spade_combine_kernel(CombineArgs a) {
           }
         }
       }
-      v.x *= m0; v.y *= m1; v.z *= m2; v.w *= m3;
+      v = make_float4(m0 ? v.x : 0.f, m1 ? v.y : 0.f, m2 ? v.z : 0.f, m3 ? v.w : 0.f);
       __stcs(reinterpret_cast<float4*>(a.dx + off + c * 128), v);
     }
   }
@@ -507,11 +508,13 @@ __global__ void __launch_bounds__(256) pixel_pre_kernel(const float* __restrict_
 
 // dxn = dpre*gam (over `pre_dxn`), dgam = dpre*(x*sc+sh) (over `gam_dgam`); per-channel sums
 //   sums[0][c] = sum dxn*x, sums[1][c] = sum dxn, sums[2][c] = sum dgam     (fp64, accumulated)
+// over the valid pixels only: the padding rows of the last tile hold whatever the producers left there (dpre comes from
+// the data-gradient engine, which never writes them), so they are selected away and written back as zeros.
 // Same mapping as the combine kernel: warp w owns channels w, w+8, ..., a lane owns 4 pixels of the tile.
 __global__ void __launch_bounds__(256) pixel_mod_bwd_kernel(const float* __restrict__ dpre, const float* __restrict__ x,
                                                             long x_bstride, const float* __restrict__ scsh,
                                                             float* __restrict__ gam_dgam, float* __restrict__ dxn,
-                                                            double* __restrict__ sums, int B, int T) {
+                                                            double* __restrict__ sums, int B, int T, int HW) {
   __shared__ float s_acc[3 * kWC];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int i = threadIdx.x; i < 3 * kWC; i += blockDim.x) s_acc[i] = 0.f;
@@ -521,12 +524,15 @@ __global__ void __launch_bounds__(256) pixel_mod_bwd_kernel(const float* __restr
     const int b = tile / T, ti = tile - b * T;
     const long off = static_cast<long>(tile) * kWC * 128 + lane * 4;
     const long xoff = static_cast<long>(b) * x_bstride + static_cast<long>(ti) * kWC * 128 + lane * 4;
+    const int p = ti * 128 + lane * 4;
+    const bool v0 = p < HW, v1 = p + 1 < HW, v2 = p + 2 < HW, v3 = p + 3 < HW;
+    auto valid4 = [&](float4 t) { return make_float4(v0 ? t.x : 0.f, v1 ? t.y : 0.f, v2 ? t.z : 0.f, v3 ? t.w : 0.f); };
 #pragma unroll 4
     for (int c = warp; c < kWC; c += 8) {
       const float sc = scsh[c], sh = scsh[kWC + c];
-      const float4 d = __ldcs(reinterpret_cast<const float4*>(dpre + off + c * 128));
-      const float4 xv = __ldcs(reinterpret_cast<const float4*>(x + xoff + c * 128));
-      const float4 g = __ldcs(reinterpret_cast<const float4*>(gam_dgam + off + c * 128));
+      const float4 d = valid4(__ldcs(reinterpret_cast<const float4*>(dpre + off + c * 128)));
+      const float4 xv = valid4(__ldcs(reinterpret_cast<const float4*>(x + xoff + c * 128)));
+      const float4 g = valid4(__ldcs(reinterpret_cast<const float4*>(gam_dgam + off + c * 128)));
       const float4 dx = make_float4(d.x * g.x, d.y * g.y, d.z * g.z, d.w * g.w);
       const float4 dg = make_float4(d.x * fmaf(xv.x, sc, sh), d.y * fmaf(xv.y, sc, sh), d.z * fmaf(xv.z, sc, sh),
                                     d.w * fmaf(xv.w, sc, sh));
@@ -745,7 +751,8 @@ int hg_spade_pixel_mod_bwd(const float* dpre, const float* x, long x_bstride, co
   const int T = (Hg * Wg + 127) / 128;
   int grid = hg::num_sms() * 4;
   if (grid > B * T) grid = B * T;
-  hg::pixel_mod_bwd_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(dpre, x, x_bstride, scsh, gam_dgam, dxn, sums, B, T);
+  hg::pixel_mod_bwd_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(dpre, x, x_bstride, scsh, gam_dgam, dxn, sums, B, T,
+                                                                               Hg * Wg);
   return hg::check_launch("hg_spade_pixel_mod_bwd");
 }
 

@@ -143,12 +143,18 @@ int hg_spade_bwd_wgrad(const float* dout, const float* x, long x_bstride, const 
  *                          mod [B,2,Cout] or NULL (g1 = 1, g0 = 0); sums [B,2,Cout] fp64 += (sum out, sum out*aux);
  *                          pixel_major: out is [B,HW,Cout] instead (Cout == 128 only).
  * hg_wgrad_blocked:        dw[256, Cx] = sum_{b,p} dout[b,:,p] (x) lrelu(x*g1+g0)[b,:,p], x with Cx in {128,256} channels
- *                          (mod NULL: g1 = 1, g0 = 0), dbias[256] = sum dout; workspace as hg_spade_bwd_wgrad.
+ *                          (mod [B,2,256] with rows past Cx unused, or NULL: g1 = 1, g0 = 0), dbias[256] = sum dout;
+ *                          padding rows of both operands are ignored; workspace as hg_spade_bwd_wgrad.
  * hg_spade_a1:             A1[B,T,128,128] = relu(bilinear_up(p_lr) + p_bias), the hidden layer of the gamma/beta MLP.
  * hg_spade_pixel_pre:      bet_pre <- (x*sc + sh)*gam + bet_pre                (scsh = [2,C]).
- * hg_spade_pixel_mod_bwd:  dxn = dpre*gam, gam_dgam <- dpre*(x*sc+sh); sums[3,C] fp64 += (sum dxn*x, sum dxn, sum dgam).
+ * hg_spade_pixel_mod_bwd:  dxn = dpre*gam, gam_dgam <- dpre*(x*sc+sh); sums[3,C] fp64 += (sum dxn*x, sum dxn, sum dgam)
+ *                          over the valid pixels.
  * hg_bilinear_adjoint:     dp[b*Rh*Rw + s, 0:128] = adjoint of the align_corners=False bilinear up-sample applied to
- *                          da1 [B,HW,128] (pixel-major); dp rows have stride dp_stride floats. */
+ *                          da1 [B,HW,128] (pixel-major); dp rows have stride dp_stride floats.
+ * Padding rows (pixels past HW in the last tile of a sample) may hold anything, NaN included: every kernel here ignores them
+ * in its inputs, except hg_spade_pixel_pre, which computes them like valid rows.  The engine (conv1x1 forward / backward)
+ * leaves them unwritten in its tile-blocked outputs; hg_spade_a1, hg_spade_pixel_mod_bwd and hg_spade_bwd_combine write
+ * zeros there. */
 int hg_conv1x1_blocked(const float* x, int Cin, const void* wimg, const float* bias, float* out, int B, int Hg, int Wg,
                        int passes, void* stream);
 /* act (0 LeakyReLU/ReLU, 1 sine/cosine) selects the mask; ascale [B,256] scales g per (sample, channel) before the product
@@ -163,7 +169,7 @@ int hg_conv1x1_blocked_bwd(const float* g, const float* g2, const float* aux, co
 int hg_act_conv1x1_blocked(const float* x, const float* x2, const float* mod, int act, const void* wimg, const float* bias,
                            float* out, int B, int Hg, int Wg, int passes, void* stream);
 /* The same engine with every option exposed: K = 256 or 512 input channels from one or two tile-blocked sources, a
- * modulation table per source (mod / mod2 [B,2,256]; null = identity), act 0 = LeakyReLU(slope) / 1 = sine, residual add,
+ * modulation table per source (mod / mod2 [B,2,256]; null = identity), act 0 = LeakyReLU(slope), 0 <= slope <= 1 / 1 = sine, residual add,
  * next-layer BatchNorm statistics, ToRGB accumulation -- one output half (256 channels) of a layer whose width was
  * zero-padded to 512: hidden_dim 384 (configs/map3d.py:61) and 420 (:254, the released checkpoint) run on it. */
 int hg_blocked_conv_wide(const float* x, const float* x2, const float* mod, const float* mod2, int act, float slope,
